@@ -2,6 +2,7 @@
 """Benchmark of the UniDepthV2.infer() hot path (see BASELINE.json / SURVEY.md section 8d).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|torch-gpu] [--workload default|hires|v1]
+                    [--dump-outputs DIR]
 
 A "step" = one `infer` pass over one batch of synthetic uint8 RGB.  Workloads (BASELINE.json `configs`):
   default  configs[1]/[2]: ViT-L/14, 8 x 3x480x640 per GPU  (the configuration the metric is quoted on)
@@ -14,6 +15,8 @@ depth + intrinsics inside the timed region (`e2e_full`: D2H of the whole seven-t
 /root/reference does not exist on the GPU box).  `--impl torch-gpu` is an INFORMATIVE extra arm, never the
 product: the same oracle port run by stock PyTorch on the GPU under fp16 autocast (what the reference itself does
 on a GPU, unidepthv2.py:239-241) -- the "kernel to beat on the same box" of BASELINE.md section 4.
+`--dump-outputs DIR` writes the outputs of the last timed step as DIR/<name>.npy (see dump_outputs) so that two builds
+can be compared output for output: weights and inputs are seeded, identical from run to run with the same arguments.
 """
 from __future__ import annotations
 
@@ -29,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no bytecode cache next to the sources
 
 import torch  # noqa: E402
 
@@ -62,6 +66,27 @@ def oracle_for(workload):
         return make_v1_state_dict, lambda sd, cfg, rgb: O1.infer_v1(sd, copy.deepcopy(cfg), rgb)
     import unidepth_oracle as O
     return make_state_dict, lambda sd, cfg, rgb: O.infer_v2(sd, copy.deepcopy(cfg), rgb)
+
+
+DUMP_BYTES = 63 * 10**6          # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out, path):
+    """Write each output tensor of one infer as <path>/<name>.npy in float32, at most DUMP_BYTES in all.  Smallest first,
+    each output gets an equal share of the budget still left; one larger than its share is replaced by a fixed sample of
+    its elements (flattened, at indices drawn with seed 0 and sorted), so runs with the same arguments sample the same
+    elements."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    left, n = DUMP_BYTES // 4, len(out)
+    for name, t in sorted(out.items(), key=lambda kv: kv[1].numel()):
+        a = t.detach().float().cpu()
+        cap = left // n
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+        left, n = left - a.numel(), n - 1
 
 
 def measured_peaks():
@@ -166,8 +191,10 @@ def run_reference(args, rank, world):
         oracle_infer(sd, cfg, x)
     t0 = time.perf_counter()
     for _ in range(steps):
-        oracle_infer(sd, cfg, x)
+        out = oracle_infer(sd, cfg, x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     val = steps * b / dt
     sample = (f"{steps} steps x batch {b} of the workload's {W['batch']}-image batch, torch fp32, {cores} threads "
               f"(best of 32/64/128) of {os.cpu_count()} cores")
@@ -214,6 +241,8 @@ def run_torch_gpu(args, rank, world):
     e.record()
     torch.cuda.synchronize()
     ms = s.elapsed_time(e)
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     torch.set_num_threads(min(64, os.cpu_count()))
     ref = oracle_infer(sd, cfg, rgb[:1])
     d, dr = out["depth"][:1].float().cpu(), ref["depth"]
@@ -242,7 +271,11 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="images per GPU per step (default: the workload's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--fuse-ln", action="store_true", help="A/B: fold norm1 / norm2 into the qkv / fc1 GEMMs (UniDepthV2.fuse_ln)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    "(float32; rank 0's images; a fixed seeded sample of an output above its share of 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -396,6 +429,8 @@ def main():
         sampler.start()
     ms = timed(step_device, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(last_out["v"], args.dump_outputs)
     step_e2e = make_e2e(False)
     for _ in range(2):
         step_e2e()

@@ -21,20 +21,21 @@ sys.path[:0] = [REF, os.path.join(HERE, "ref_shims"), HERE]
 from fixture import make_state_dict, param_shapes  # noqa: E402
 
 CASES = [
-    # name, config, seed, (B,H,W), resolution_level
+    # name, config, seed, (B,H,W), resolution_level[, strides as in BIG_CASES; default (1, 1, 4)]
     ("vits_120x160", "config_v2_vits14.json", 0, (1, 120, 160), None),
-    ("vits_pad_96x288_rl3", "config_v2_vits14.json", 1, (2, 96, 288), 3),
+    ("vits_pad_96x288_rl3", "config_v2_vits14.json", 1, (2, 96, 288), 3, (1, 2, 16)),
     ("vitb_112x160", "config_v2_vitb14.json", 2, (1, 112, 160), None),
 ]
 # The benchmark configuration itself (BASELINE.json configs[1]: ViT-L/14, 3x480x640), full depth, one image.
 # Takes a few minutes on CPU, so it is generated on request:  python oracle/make_golden.py vitl
-# Stored: depth and intrinsics in full; the other maps every 4th pixel; depth_features every 8th channel.
+# Stored: intrinsics in full; depth every 2nd pixel; the other maps every 4th pixel; depth_features every 32nd channel.
 # `python oracle/make_golden.py vitl` also writes BASELINE configs[4]'s shape (3x1024x1536 -> 644x952, 3129 tokens) at full
-# depth: depth every 2nd pixel, the other maps every 8th.
+# depth: depth every 4th pixel, the other maps every 16th, depth_features every 32nd channel.
+# The strides keep every file under 1 MB.
 BIG_CASES = [
     # name, config, seed, (B,H,W), resolution_level, (depth stride, spatial stride, depth_features channel stride)
-    ("vitl_480x640", "config_v2_vitl14.json", 0, (1, 480, 640), None, (1, 4, 8)),
-    ("vitl_1024x1536", "config_v2_vitl14.json", 3, (1, 1024, 1536), None, (2, 8, 16)),
+    ("vitl_480x640", "config_v2_vitl14.json", 0, (1, 480, 640), None, (2, 4, 32)),
+    ("vitl_1024x1536", "config_v2_vitl14.json", 3, (1, 1024, 1536), None, (4, 16, 32)),
 ]
 
 
@@ -70,7 +71,7 @@ def main():
         rgb = seeded_rgb(shape, seed)
         out = model.infer(rgb)
         arrays = {k: v.detach().cpu().numpy() for k, v in out.items()}
-        # depth_features is large; keep every 4th channel (the restatement is checked on those)
+        # depth_features is large; keep every sc_-th channel (the restatement is checked on those)
         arrays["depth_features"] = arrays["depth_features"][:, ::sc_]
         arrays["depth"] = arrays["depth"][:, :, ::sd_, ::sd_]
         for k in ("confidence", "radius", "points", "rays"):

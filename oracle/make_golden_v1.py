@@ -69,9 +69,11 @@ def main():
             K = torch.tensor([[[720.0, 0.0, 610.0], [0.0, 725.0, 180.0], [0.0, 0.0, 1.0]]])
         out = model.infer(rgb, K.clone() if K is not None else None, skip_camera=skip)
         arrays = {k: v.detach().cpu().numpy() for k, v in out.items()}
+        # every 4th pixel of the points and every 2nd of the depth keep each file under 1 MB
         arrays["points"] = arrays["points"][:, :, ::4, ::4]
+        arrays["depth"] = arrays["depth"][:, :, ::2, ::2]
         meta = dict(config="config_v1_cnvnxtl.json", seed=seed, shape=list(shape), with_k=with_k, skip_camera=skip,
-                    strides=dict(points=4))
+                    strides=dict(points=4, depth=2))
         if K is not None:
             arrays["K_in"] = K.numpy()
         np.savez_compressed(os.path.join(out_dir, name + ".npz"), __meta__=json.dumps(meta), **arrays)

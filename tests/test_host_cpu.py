@@ -31,7 +31,11 @@ def test_library_exports_every_header_symbol():
         assert hasattr(lib, n), f"libudb.so does not export {n}"
     assert set(_cabi.EXPORTS) == names, (set(_cabi.EXPORTS) ^ names)
     assert _cabi.lib().udb_version() == 1
-    assert _cabi.lib().udb_launch_count() == 0
+    # a freshly loaded library has launched nothing; checked in a new process because GPU tests earlier in this one
+    # have already advanced the counter
+    fresh = subprocess.check_output([sys.executable, "-c", "import sys; sys.path.insert(0, sys.argv[1]); "
+                                     "from unidepth_b200 import _cabi; print(_cabi.lib().udb_launch_count())", ROOT], text=True)
+    assert int(fresh) == 0
 
 
 def test_ctypes_structs_match_c_layout():

@@ -195,7 +195,8 @@ def test_v1_oracle_matches_reference_golden(name, golden_dir):
     assert set(out) == {"intrinsics", "points", "depth"}
     for k in ("intrinsics", "depth", "points"):
         ref = torch.from_numpy(z[k])
-        got = out[k][:, :, ::meta["strides"]["points"], ::meta["strides"]["points"]] if k == "points" else out[k]
+        s = meta["strides"].get(k, 1)
+        got = out[k][:, :, ::s, ::s] if k in ("depth", "points") else out[k]
         assert got.shape == ref.shape, (k, got.shape, ref.shape)
         floor = 0.1 * ref.abs().mean().item()
         err = ((got - ref).abs() / ref.abs().clamp(min=floor)).max().item()

@@ -247,8 +247,8 @@ V1_MEASURED = {
 }
 
 
-def _check_v1(out, ref_depth, ref_K, ref_pts, tag, pts_stride=1):
-    d, dr = out["depth"].float().cpu(), ref_depth
+def _check_v1(out, ref_depth, ref_K, ref_pts, tag, pts_stride=1, depth_stride=1):
+    d, dr = out["depth"].float().cpu()[:, :, ::depth_stride, ::depth_stride], ref_depth
     rel = (d - dr).abs() / dr
     k, kr = out["intrinsics"].cpu(), ref_K
     kerr = max(((k[:, i, j] - kr[:, i, j]).abs() / kr[:, i, j].abs()).max().item() for i, j in ((0, 0), (1, 1), (0, 2), (1, 2)))
@@ -269,7 +269,7 @@ def test_v1_infer_against_reference_golden(name, golden_dir):
     out = m.infer(rgb, K, skip_camera=meta["skip_camera"])
     assert set(out) == {"intrinsics", "points", "depth"}
     _check_v1(out, torch.from_numpy(z["depth"]), torch.from_numpy(z["intrinsics"]), torch.from_numpy(z["points"]), "golden_" + name,
-              meta["strides"]["points"])
+              meta["strides"]["points"], meta["strides"]["depth"])
     # graph replay and eager agree bit for bit; a batch returns each image's single-image result
     again = m.infer(rgb, K, skip_camera=meta["skip_camera"])
     assert all(torch.equal(again[k], out[k]) for k in out)
