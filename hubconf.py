@@ -2,8 +2,9 @@
 
     model = torch.hub.load(<this repo>, "UniDepth", version="v2", backbone="vitl14", pretrained=True, source="local")
 
-UniDepthV2 (ViT-L/B/S) and UniDepthV1 with the ConvNeXt-L encoder are implemented on the B200 path (SURVEY.md section 8);
-the other entries the reference lists raise NotImplementedError instead of silently loading something else."""
+UniDepthV2 (ViT-L/B/S) and UniDepthV1 with the ConvNeXt-L encoder load through this entry; UniDepthV1 with ViT-L runs on the
+B200 path through `UniDepthV1(config_v1_vitl14.json)` but not through the hub entry yet.  The other entries the reference
+lists raise NotImplementedError instead of silently loading something else."""
 dependencies = ["torch"]
 
 import json
@@ -21,6 +22,10 @@ def UniDepth(version="v2", backbone="vitl14", pretrained=True):
         raise AssertionError(f"version must be one of {sorted(set(_SUPPORTED) | set(_KNOWN_ELSEWHERE))}")
     if backbone not in _SUPPORTED.get(version, ()):
         if backbone in _KNOWN_ELSEWHERE.get(version, ()):
+            if version == "v1":
+                raise NotImplementedError(f"UniDepth v1 {backbone}: not available through the hub entry yet; build it with "
+                                          f"UniDepthV1(json.load(open('unidepth_b200/configs/config_v1_{backbone}.json'))) "
+                                          "or UniDepthV1.from_pretrained(...)")
             raise NotImplementedError(f"UniDepth {version} {backbone} is not part of the B200 inference path")
         raise AssertionError(f"backbone for version {version} must be one of {list(_SUPPORTED.get(version, ()))}")
     cfg_path = os.path.join(_HERE, "unidepth_b200", "configs", f"config_{version}_{backbone}.json")

@@ -321,6 +321,14 @@ typedef struct udb_v1_preprocess_t {
   void* patches;
 } udb_v1_preprocess_t;
 int udb_v1_preprocess(const udb_v1_preprocess_t* p, void* stream);
+/* The same pre-processing for the DINOv2 ViT encoder (V1 with dinov2_vit*14): 14x14 stride-14 patch rows
+ * [B*gh*gw, 640] f16 (column c*196 + py*14 + px, 588 used, the rest zero; gh = net_h/14), the operand layout of the
+ * patch-embedding GEMM. */
+int udb_v1_preprocess_vit(const udb_v1_preprocess_t* p, void* stream);
+/* ViT tap after one encoder block (unidepthv1.py:322-326, decoder.py:371-374).  x: f32 residual stream [B, T, D] (row 0 =
+ * cls).  dst [B, T-1, D] f16: f16(x[b,1+n,:] + x[b,0,:]) when `first`, else the element-wise max of dst and that (the
+ * running max over a block range).  cls (may be NULL): x[b,0,:] copied to [B, D] f32.  D % 8 == 0, 16-byte aligned. */
+int udb_vit_tap_f16(const float* x, void* dst, float* cls, int32_t B, int32_t T, int32_t D, int32_t first, void* stream);
 
 /* LayerNorm over the last dim for widths that are multiples of 64 up to 1536 (ConvNeXt channel LayerNorm / LayerNorm2d,
  * convnext.py:214,252-263; decoder LayerNorms).  in row r at in + r*ld_in (+ add[(r % add_mod)*dim ..] when add != NULL:
@@ -564,6 +572,13 @@ typedef struct udb_v1_config_t {
 } udb_v1_config_t;
 
 int udb_v1_create(const udb_v1_config_t* cfg, udb_engine_v1** out);
+/* UniDepthV1 with a DINOv2 ViT encoder (dinov2_vit*14, e.g. config_v1_vitl14.json): cfg->depths hold the lengths of
+ * the four block ranges the decoder max-stacks (ViT-L with output_idx 5,12,18,24: 5,7,6,6), cfg->dims the embedding
+ * width four times, enc_heads the encoder's heads (64-wide).  The network shape must be a multiple of 14.  Encoder
+ * operands: patch_w [D, 640] f16 (588 used), patch_b, cls [D], pos [1 + gh*gw, D] f32 (the position table already
+ * resampled to the network grid), blocks.<i>.{n1w,n1b,qkv_w,qkv_b,proj_w,proj_b,ls1,n2w,n2b,fc1_w,fc1_b,fc2_w,fc2_b,ls2}
+ * as in the V2 engine's default mode; the decoder's are the ConvNeXt model's. */
+int udb_v1_create_vit(const udb_v1_config_t* cfg, int32_t enc_heads, udb_engine_v1** out);
 void udb_v1_destroy(udb_engine_v1* e);
 int udb_v1_set_weight(udb_engine_v1* e, const char* name, const void* dev_ptr, const int64_t* shape, int32_t ndim,
                       int32_t dtype);

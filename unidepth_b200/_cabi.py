@@ -210,6 +210,8 @@ EXPORTS = {
     "udb_infer_v2": (i32, [vp, C.POINTER(InferArgs), vp]),
     # UniDepthV1 operators + engine
     "udb_v1_preprocess": (i32, [C.POINTER(V1Preprocess), vp]),
+    "udb_v1_preprocess_vit": (i32, [C.POINTER(V1Preprocess), vp]),
+    "udb_vit_tap_f16": (i32, [vp, vp, vp, i32, i32, i32, i32, vp]),
     "udb_layernorm_any": (i32, [C.POINTER(LayerNormAny), vp]),
     "udb_dwconv7_nhwc_f16": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, vp]),
     "udb_max_accum_f16": (i32, [vp, vp, i64, i32, vp]),
@@ -228,6 +230,7 @@ EXPORTS = {
     "udb_v1_mean_maps": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]),
     "udb_v1_postprocess": (i32, [C.POINTER(V1Postprocess), vp]),
     "udb_v1_create": (i32, [C.POINTER(V1Config), C.POINTER(vp)]),
+    "udb_v1_create_vit": (i32, [C.POINTER(V1Config), i32, C.POINTER(vp)]),
     "udb_v1_destroy": (None, [vp]),
     "udb_v1_set_weight": (i32, [vp, C.c_char_p, vp, C.POINTER(i64), i32, i32]),
     "udb_v1_set_scalar": (i32, [vp, C.c_char_p, C.c_double]),

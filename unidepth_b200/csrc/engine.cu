@@ -135,46 +135,10 @@ static int run(udb_engine* e, const udb_infer_args_t& a, const udb_geometry_t& g
     __half* qkv = ar.h(BT * 3 * D * sx);
     __half* att = ar.h(BT * D * sx);
     __half* mid = ar.h(BT * 4 * D * sx);
-    const int kx = sp ? 3 : 1;          // logical K multiplier of a split operand
+    const VitScratch vs{h, qkv, att, mid, x16, stats, ln_parts, ln_pc};
     int tap = 0;
     for (int i = 0; i < cf.depth; ++i) {
-      const std::string b = idx("blocks.%d.", i);
-      // a weight packed for another mode (or transposed) must be refused, not read with the wrong leading dimension
-      c.expect2(b + (fuse ? "qkv_wf" : "qkv_w"), 3 * D, D * kx);
-      c.expect2(b + (fuse ? "fc1_wf" : "fc1_w"), 4 * D, D * kx);
-      c.expect2(b + "proj_w", D, D * kx);
-      c.expect2(b + "fc2_w", D, 4 * D * kx);
-      if (fuse) {
-        Ctx::G q{x16, c.H(b + "qkv_wf"), static_cast<int>(BT), 3 * D, D};
-        q.bias = c.F(b + "qkv_c2"); q.ln_stats_in = stats; q.ln_c1 = c.F(b + "qkv_c1"); q.ln_parts = ln_parts; q.ln_part_cols = ln_pc;
-        q.ln_eps = 1e-6f; q.out = qkv; c.gemm(q);
-      } else {
-        c.layernorm(x, 1, h, 0, c.F(b + "n1w"), c.F(b + "n1b"), static_cast<int>(BT), D, 1e-6f, 0, 0, 0, 0, sp ? D : 0);
-        Ctx::G q{h, c.H(b + "qkv_w"), static_cast<int>(BT), 3 * D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
-        q.bias = c.F(b + "qkv_b"); q.out = qkv; q.ldc = 3 * D * sx; q.out_split = sp ? 3 * D : 0; c.gemm(q);
-      }
-      c.attention(qkv, qkv, qkv, att, B, cf.enc_heads, T, T, 3 * D * sx, 3 * D * sx, 3 * D * sx, D * sx, 0, D, 2 * D, 0.125f,
-                  sp ? 3 * D : 0, sp ? D : 0);
-      { Ctx::G q{att, c.H(b + "proj_w"), static_cast<int>(BT), D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
-        q.bias = c.F(b + "proj_b"); q.gamma = c.F(b + "ls1");
-        q.resid = x; q.resid_f32 = 1; q.out = x; q.out_f32 = 1;
-        if (fuse) { q.out2 = x16; q.out2_leaky = 0; q.ln_stats_out = stats; q.ln_parts = ln_parts; q.ln_part_cols = ln_pc; }
-        c.gemm(q); }
-      if (fuse) {
-        Ctx::G q{x16, c.H(b + "fc1_wf"), static_cast<int>(BT), 4 * D, D};
-        q.bias = c.F(b + "fc1_c2"); q.ln_stats_in = stats; q.ln_c1 = c.F(b + "fc1_c1"); q.ln_parts = ln_parts; q.ln_part_cols = ln_pc;
-        q.ln_eps = 1e-6f; q.act = UDB_ACT_GELU; q.out = mid; c.gemm(q);
-      } else {
-        c.layernorm(x, 1, h, 0, c.F(b + "n2w"), c.F(b + "n2b"), static_cast<int>(BT), D, 1e-6f, 0, 0, 0, 0, sp ? D : 0);
-        Ctx::G q{h, c.H(b + "fc1_w"), static_cast<int>(BT), 4 * D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
-        q.bias = c.F(b + "fc1_b"); q.act = UDB_ACT_GELU;
-        q.out = mid; q.ldc = 4 * D * sx; q.out_split = sp ? 4 * D : 0; c.gemm(q);
-      }
-      { Ctx::G q{mid, c.H(b + "fc2_w"), static_cast<int>(BT), D, 4 * D * kx}; q.lda = 4 * D * sx; q.a_split_k = sp ? 4 * D : 0;
-        q.bias = c.F(b + "fc2_b"); q.gamma = c.F(b + "ls2");
-        q.resid = x; q.resid_f32 = 1; q.out = x; q.out_f32 = 1;
-        if (fuse) { q.out2 = x16; q.out2_leaky = 0; q.ln_stats_out = stats; q.ln_parts = ln_parts; q.ln_part_cols = ln_pc; }
-        c.gemm(q); }
+      vit_block(c, idx("blocks.%d.", i), x, B, T, D, cf.enc_heads, sp, fuse, vs);
       if (tap < 4 && i + 1 == cf.taps[tap]) {
         c.layernorm(x, 1, feats[tap], 0, c.F("norm_w"), c.F("norm_b"), static_cast<int>(BN), D, 1e-5f, N, T, 1);
         c.layernorm(x, 1, clss[tap], 1, c.F("norm_w"), c.F("norm_b"), B, D, 1e-5f, 1, T, 0);

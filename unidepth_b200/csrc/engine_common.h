@@ -218,6 +218,68 @@ static inline float* cam_mlp(Ctx& c, const std::string& pre, const float* x, int
   return o;
 }
 
+// Scratch of vit_block, owned by the caller: h [B*T, D] (unused with fuse), qkv [B*T, 3D], att [B*T, D], mid [B*T, 4D]
+// (each x2 in split mode); x16 / stats: the f16 copy of the residual stream and its per-part LayerNorm statistics (fuse only).
+struct VitScratch {
+  __half* h;
+  __half* qkv;
+  __half* att;
+  __half* mid;
+  __half* x16;
+  float* stats;
+  int ln_parts, ln_pc;
+};
+
+// One DINOv2 block on the f32 residual stream x [B*T, D] (metadinov2/block.py:84-109): LN -> qkv -> attention (64-wide
+// heads) -> proj (ls1, +x) -> LN -> fc1 (GELU) -> fc2 (ls2, +x), with the operands blocks.<i>.* under prefix `b`.
+// sp: split-f16 precise mode (every operand a hi/lo pair, weights [N, 3K]); fuse: LayerNorm folded into qkv / fc1, whose
+// inputs are the x16 copy + statistics written by the GEMMs that update x.  Shared by the V2 engine and V1's ViT encoder.
+static inline void vit_block(Ctx& c, const std::string& b, float* x, int B, int T, int D, int heads, bool sp, bool fuse,
+                             const VitScratch& s) {
+  const size_t BT = static_cast<size_t>(B) * T;
+  const int sx = sp ? 2 : 1;
+  const int kx = sp ? 3 : 1;          // logical K multiplier of a split operand
+  const int ln_parts = s.ln_parts, ln_pc = s.ln_pc;
+  __half *h = s.h, *qkv = s.qkv, *att = s.att, *mid = s.mid, *x16 = s.x16;
+  float* stats = s.stats;
+  // a weight packed for another mode (or transposed) must be refused, not read with the wrong leading dimension
+  c.expect2(b + (fuse ? "qkv_wf" : "qkv_w"), 3 * D, D * kx);
+  c.expect2(b + (fuse ? "fc1_wf" : "fc1_w"), 4 * D, D * kx);
+  c.expect2(b + "proj_w", D, D * kx);
+  c.expect2(b + "fc2_w", D, 4 * D * kx);
+  if (fuse) {
+    Ctx::G q{x16, c.H(b + "qkv_wf"), static_cast<int>(BT), 3 * D, D};
+    q.bias = c.F(b + "qkv_c2"); q.ln_stats_in = stats; q.ln_c1 = c.F(b + "qkv_c1"); q.ln_parts = ln_parts; q.ln_part_cols = ln_pc;
+    q.ln_eps = 1e-6f; q.out = qkv; c.gemm(q);
+  } else {
+    c.layernorm(x, 1, h, 0, c.F(b + "n1w"), c.F(b + "n1b"), static_cast<int>(BT), D, 1e-6f, 0, 0, 0, 0, sp ? D : 0);
+    Ctx::G q{h, c.H(b + "qkv_w"), static_cast<int>(BT), 3 * D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
+    q.bias = c.F(b + "qkv_b"); q.out = qkv; q.ldc = 3 * D * sx; q.out_split = sp ? 3 * D : 0; c.gemm(q);
+  }
+  c.attention(qkv, qkv, qkv, att, B, heads, T, T, 3 * D * sx, 3 * D * sx, 3 * D * sx, D * sx, 0, D, 2 * D, 0.125f,
+              sp ? 3 * D : 0, sp ? D : 0);
+  { Ctx::G q{att, c.H(b + "proj_w"), static_cast<int>(BT), D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
+    q.bias = c.F(b + "proj_b"); q.gamma = c.F(b + "ls1");
+    q.resid = x; q.resid_f32 = 1; q.out = x; q.out_f32 = 1;
+    if (fuse) { q.out2 = x16; q.out2_leaky = 0; q.ln_stats_out = stats; q.ln_parts = ln_parts; q.ln_part_cols = ln_pc; }
+    c.gemm(q); }
+  if (fuse) {
+    Ctx::G q{x16, c.H(b + "fc1_wf"), static_cast<int>(BT), 4 * D, D};
+    q.bias = c.F(b + "fc1_c2"); q.ln_stats_in = stats; q.ln_c1 = c.F(b + "fc1_c1"); q.ln_parts = ln_parts; q.ln_part_cols = ln_pc;
+    q.ln_eps = 1e-6f; q.act = UDB_ACT_GELU; q.out = mid; c.gemm(q);
+  } else {
+    c.layernorm(x, 1, h, 0, c.F(b + "n2w"), c.F(b + "n2b"), static_cast<int>(BT), D, 1e-6f, 0, 0, 0, 0, sp ? D : 0);
+    Ctx::G q{h, c.H(b + "fc1_w"), static_cast<int>(BT), 4 * D, D * kx}; q.lda = D * sx; q.a_split_k = sp ? D : 0;
+    q.bias = c.F(b + "fc1_b"); q.act = UDB_ACT_GELU;
+    q.out = mid; q.ldc = 4 * D * sx; q.out_split = sp ? 4 * D : 0; c.gemm(q);
+  }
+  { Ctx::G q{mid, c.H(b + "fc2_w"), static_cast<int>(BT), D, 4 * D * kx}; q.lda = 4 * D * sx; q.a_split_k = sp ? 4 * D : 0;
+    q.bias = c.F(b + "fc2_b"); q.gamma = c.F(b + "ls2");
+    q.resid = x; q.resid_f32 = 1; q.out = x; q.out_f32 = 1;
+    if (fuse) { q.out2 = x16; q.out2_leaky = 0; q.ln_stats_out = stats; q.ln_parts = ln_parts; q.ln_part_cols = ln_pc; }
+    c.gemm(q); }
+}
+
 static inline std::string idx(const char* fmt, int i) {
   char b[64];
   snprintf(b, sizeof(b), fmt, i);

@@ -1,9 +1,10 @@
-// Whole-path engine for UniDepthV1.infer with the ConvNeXt encoder (BASELINE config 4), behind udb_v1_create /
-// udb_v1_set_weight / udb_v1_workspace_bytes / udb_infer_v1 (include/udb.h).  Host-side schedule only: it enqueues the
+// Whole-path engine for UniDepthV1.infer with the ConvNeXt encoder (BASELINE config 4) or a DINOv2 ViT encoder, behind
+// udb_v1_create / udb_v1_create_vit / udb_v1_set_weight / udb_v1_workspace_bytes / udb_infer_v1 (include/udb.h).  Host-side schedule only: it enqueues the
 // kernels of this library on the caller's stream over a bump-allocated workspace (no allocation, copy or sync inside
 // udb_infer_v1, so the call is graph-capturable).  Reference call stack it replaces:
 //   UniDepthV1.infer                 unidepth/models/unidepthv1/unidepthv1.py:288-373 (_shapes/_paddings/_preprocess/_postprocess :30-94)
 //     pixel_encoder = ConvNeXt       unidepth/models/backbones/convnext.py:459-471 (stem :371-383, stage :289-298, block :208-223)
+//                   or DINOv2        unidepth/models/backbones/dinov2.py:306-347 (all blocks, no final norm; + cls, unidepthv1.py:322-326)
 //     pixel_decoder = Decoder        unidepth/models/unidepthv1/decoder.py:364-463 (run_camera :311-343, CameraHead :85-106,
 //                                    DepthHead :195-300), layers/{attention,nystrom_attention,mlp,upsample,convnext}.py
 #include <stdlib.h>
@@ -12,6 +13,7 @@
 
 struct udb_engine_v1 : udb::EngineBase {
   udb_v1_config_t cfg;
+  int vit_heads = 0;                                  // > 0: DINOv2 ViT encoder (udb_v1_create_vit)
   std::unordered_map<std::string, size_t> ws_need;   // "B,H,W" -> bytes
 };
 
@@ -99,6 +101,47 @@ struct V1Ctx : Ctx {
 };
 
 static inline long long rup(long long v, long long m) { return (v + m - 1) / m * m; }
+
+// DINOv2 encoder of V1 (dinov2.py:306-347 with interpolate_offset 0.1, unidepthv1.py:322-326, decoder.py:371-379): 14x14
+// patches -> patch GEMM + position table -> cls row -> all blocks; after each block the (x + cls) map is max-stacked into
+// its range's level and the last four blocks' cls rows are kept (clsbuf[k]: block last - k).
+static void vit_encoder_v1(V1Ctx& c, const udb_infer_v1_args_t& a, const V1Geom& g, int vit_heads, int gh, int gw, __half* const* levels,
+                           float* const* clsbuf) {
+  const udb_v1_config_t& cf = static_cast<udb_engine_v1*>(c.e)->cfg;
+  Arena& ar = *c.ar;
+  const int B = a.B, N = gh * gw, T = N + 1, D = cf.dims[0];
+  const size_t BN = static_cast<size_t>(B) * N, BT = static_cast<size_t>(B) * T;
+  __half* patches = ar.h(BN * 640);
+  if (!c.dry) {
+    udb_v1_preprocess_t p;
+    memset(&p, 0, sizeof(p));
+    p.rgb = a.rgb; p.rgb_is_u8 = a.rgb_is_u8; p.scale255 = a.scale255; p.normalize = a.normalize; p.B = B; p.H = a.H; p.W = a.W;
+    p.rh = g.rh; p.rw = g.rw; p.pad_l = g.pad_l; p.pad_t = g.pad_t; p.net_h = cf.net_h; p.net_w = cf.net_w; p.patches = patches;
+    c.done(udb_v1_preprocess_vit(&p, c.st));
+  }
+  c.expect2("pos", T, D);                    // the position table is packed for this network grid
+  float* x = ar.f(BT * D);
+  {
+    Ctx::G q{patches, c.H("patch_w"), static_cast<int>(BN), D, 640};
+    q.bias = c.F("patch_b"); q.resid = c.F("pos"); q.resid_f32 = 1; q.ldr = D; q.out = x; q.out_f32 = 1;
+    q.rows_per_group = N; q.group_stride = T; q.row_offset = 1; q.resid_mod = N; q.resid_row_offset = 1;
+    c.expect2("patch_w", D, 640);
+    c.gemm(q);
+    const float* cls = c.F("cls");           // looked up in the dry run too, so a missing one is reported there
+    if (!c.dry && !c.rc) c.done(udb_set_cls_rows(x, cls, c.F("pos"), B, T, D, c.st));
+  }
+  const VitScratch vs{ar.h(BT * D), ar.h(BT * 3 * D), ar.h(BT * D), ar.h(BT * 4 * D), nullptr, nullptr, 0, 0};
+  int total = 0;
+  for (int l = 0; l < 4; ++l) total += cf.depths[l];
+  for (int l = 0, i = 0; l < 4; ++l)
+    for (int j = 0; j < cf.depths[l]; ++j, ++i) {
+      vit_block(c, idx("blocks.%d.", i), x, B, T, D, vit_heads, false, false, vs);
+      const int from_end = total - 1 - i;
+      if (!c.dry && !c.rc) c.done(udb_vit_tap_f16(x, levels[l], from_end < 4 ? clsbuf[from_end] : nullptr, B, T, D, j == 0, c.st));
+      if (i == 0) c.tap("enc_block0", x, sizeof(float) * BT * D);
+    }
+  c.tap("enc_last", x, sizeof(float) * BT * D);
+}
 
 // Single-head (head dim = D) attention block with a separate context (decoder.py:225-236 aggregate_16 / prompt_camera),
 // computed densely: S = q k^T (GEMM) -> row softmax -> P v (GEMM with v^T as the K-major operand).
@@ -203,9 +246,10 @@ static int run_v1(udb_engine_v1* e, const udb_infer_v1_args_t& a, Arena& ar, voi
   c.e = e; c.ar = &ar; c.st = st; c.dry = ar.dry;
   const int B = a.B, net_h = cf.net_h, net_w = cf.net_w, hid = cf.hidden;
   const V1Geom g = v1_geometry(a.H, a.W, net_h, net_w);
-  int sh[4], sw[4];
-  sh[0] = (net_h - 4) / 4 + 1; sw[0] = (net_w - 4) / 4 + 1;
-  for (int i = 1; i < 4; ++i) { sh[i] = sh[i - 1] / 2; sw[i] = sw[i - 1] / 2; }
+  const bool vit = e->vit_heads > 0;
+  int sh[4], sw[4];                 // level grids: the ConvNeXt pyramid, or the ViT patch grid four times
+  sh[0] = vit ? net_h / 14 : (net_h - 4) / 4 + 1; sw[0] = vit ? net_w / 14 : (net_w - 4) / 4 + 1;
+  for (int i = 1; i < 4; ++i) { sh[i] = vit ? sh[0] : sh[i - 1] / 2; sw[i] = vit ? sw[0] : sw[i - 1] / 2; }
   Stage stage;
 
   // ---- pre-processing + stem (convnext.py:371-383: conv k4 s4 as an im2col GEMM, then LayerNorm2d)
@@ -224,7 +268,12 @@ static int run_v1(udb_engine_v1* e, const udb_infer_v1_args_t& a, Arena& ar, voi
     if (k != 4) { set_error("udb_infer_v1: the encoder needs at least four blocks"); return 1; }
   }
   for (int k = 0; k < 4; ++k) clsbuf[k] = ar.f(static_cast<size_t>(B) * cls_dim[k]);     // clsbuf[k]: block (last - k)
-  {
+  if (vit) {
+    stage.next("udb_v1:vit_encoder");
+    const size_t enc_mark = ar.mark();
+    vit_encoder_v1(c, a, g, e->vit_heads, sh[0], sw[0], levels, clsbuf);
+    ar.release(enc_mark);
+  } else {
     const size_t enc_mark = ar.mark();
     const long long n0 = static_cast<long long>(B) * sh[0] * sw[0];
     __half* patches = ar.h(n0 * 64);
@@ -275,7 +324,7 @@ static int run_v1(udb_engine_v1* e, const udb_infer_v1_args_t& a, Arena& ar, voi
     ar.release(enc_mark);
   }
 
-  // ---- decoder: common grid = second-smallest level (decoder.py:381-392), adapters (:395-408)
+  // ---- decoder: common grid = second-smallest level (decoder.py:381-392; the ViT's one grid), adapters (:395-408)
   stage.next("udb_v1:adapters");
   const int hc = sh[2], wc = sw[2], nq = hc * wc;
   const long long Rq = static_cast<long long>(B) * nq;
@@ -507,6 +556,25 @@ int udb_v1_create(const udb_v1_config_t* cfg, udb_engine_v1** out) {
   udb_engine_v1* e = new udb_engine_v1();
   e->cfg = *cfg;
   *out = e;
+  return 0;
+}
+
+int udb_v1_create_vit(const udb_v1_config_t* cfg, int32_t enc_heads, udb_engine_v1** out) {
+  if (!cfg || !out) { set_error("udb_v1_create_vit: null argument"); return 1; }
+  const int D = cfg->dims[0];
+  for (int i = 0; i < 4; ++i)
+    if (cfg->dims[i] != D || cfg->depths[i] <= 0) {
+      set_error("udb_v1_create_vit: range %d (depth %d, width %d): the four widths must equal the embedding width and every "
+                "range needs a block", i, cfg->depths[i], cfg->dims[i]);
+      return 1;
+    }
+  if (D <= 0 || D % 64 || D > 1536 || enc_heads <= 0 || D / enc_heads != 64 || D % enc_heads) {
+    set_error("udb_v1_create_vit: encoder width %d / heads %d: needs 64-wide heads and a width up to 1536", D, enc_heads);
+    return 1;
+  }
+  if (cfg->net_h % 14 || cfg->net_w % 14) { set_error("udb_v1_create_vit: network shape %dx%d is not a multiple of 14", cfg->net_h, cfg->net_w); return 1; }
+  if (udb_v1_create(cfg, out)) return 1;
+  (*out)->vit_heads = enc_heads;
   return 0;
 }
 

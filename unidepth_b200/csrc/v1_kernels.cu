@@ -62,25 +62,28 @@ __device__ __forceinline__ AAxis aa_axis(int i, int in_size, float scale) {
 
 // ------------------------------------------------------------------------------------------------------------------
 // V1 pre-processing (unidepthv1.py:49-63,298-317): u8 / f32 NCHW -> /255 -> ImageNet normalise -> antialiased bilinear
-// to (rh, rw) -> zero pad to the fixed network shape -> 4x4 stride-4 patch rows [B*gh*gw, 64] f16 (48 used:
-// column c*16 + py*4 + px, the stem conv's im2col, convnext.py:371-383).
+// to (rh, rw) -> zero pad to the fixed network shape -> PxP stride-P patch rows [B*gh*gw, LD] f16 (column
+// c*P*P + py*P + px, 3*P*P used, the rest zero).  P = 4, LD = 64: the ConvNeXt stem conv's im2col (convnext.py:371-383);
+// P = 14, LD = 640: the DINOv2 patch embedding's (V2's patch-GEMM operand layout).
 // ------------------------------------------------------------------------------------------------------------------
+template <int P, int LD>
 __global__ void __launch_bounds__(256) v1_preprocess_kernel(const udb_v1_preprocess_t p, int gh, int gw, float sh, float sw) {
-  const long long total = (long long)p.B * gh * gw * 8;   // 8 x (8 columns) per patch row
+  constexpr int NV = LD / 8;                              // 8-column vectors per patch row
+  const long long total = (long long)p.B * gh * gw * NV;
   const float mean[3] = {0.485f, 0.456f, 0.406f};
   const float stdv[3] = {0.229f, 0.224f, 0.225f};
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
-    const int v8 = (int)(idx & 7);
-    const long long row = idx >> 3;
+    const int v8 = (int)(idx % NV);
+    const long long row = idx / NV;
     const int gx = (int)(row % gw), gy = (int)((row / gw) % gh), b = (int)(row / ((long long)gw * gh));
     float val[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int col = v8 * 8 + j;
       float acc = 0.f;
-      if (col < 48) {
-        const int c = col >> 4, py = (col >> 2) & 3, px = col & 3;
-        const int Y = gy * 4 + py - p.pad_t, X = gx * 4 + px - p.pad_l;     // position in the resized image
+      if (col < 3 * P * P) {
+        const int c = col / (P * P), py = (col / P) % P, px = col % P;
+        const int Y = gy * P + py - p.pad_t, X = gx * P + px - p.pad_l;     // position in the resized image
         if (Y >= 0 && Y < p.rh && X >= 0 && X < p.rw) {
           const AAxis ay = aa_axis(Y, p.H, sh), ax = aa_axis(X, p.W, sw);
           for (int jy = 0; jy < ay.xsize; ++jy) {
@@ -99,7 +102,7 @@ __global__ void __launch_bounds__(256) v1_preprocess_kernel(const udb_v1_preproc
       }
       val[j] = acc;
     }
-    *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.patches) + row * 64 + v8 * 8) =
+    *reinterpret_cast<uint4*>(reinterpret_cast<__half*>(p.patches) + row * LD + v8 * 8) =
         make_uint4(pack_half2(val[0], val[1]), pack_half2(val[2], val[3]), pack_half2(val[4], val[5]), pack_half2(val[6], val[7]));
   }
 }
@@ -271,6 +274,38 @@ __global__ void __launch_bounds__(256) max_accum_kernel(const uint4* __restrict_
       for (int j = 0; j < 4; ++j) sh[j] = __hmax2(sh[j], dh[j]);
     }
     dst[i] = s;
+  }
+}
+
+// ViT tap after one block (unidepthv1.py:322-326 + decoder.py:371-374): dst[b, n, :] = f16(x[b, 1+n, :] + x[b, 0, :]) on the
+// first block of a range, max(dst, that) on the later ones; f16 rounding is monotone, so the running f16 max equals one
+// rounding of the f32 max.  cls (optional): the f32 cls row x[b, 0, :] -> [B, D].  One thread per 8 channels (16-byte stores).
+__global__ void __launch_bounds__(256) vit_tap_kernel(const float* __restrict__ x, uint4* __restrict__ dst, float* __restrict__ cls,
+                                                      int N, int D, long long total, int first) {
+  const int dv = D >> 3;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int c8 = (int)(i % dv);
+    const long long bn = i / dv;
+    const long long b = bn / N, n = bn % N;
+    const float* xc = x + b * (N + 1) * D + c8 * 8;
+    const float4* pr = reinterpret_cast<const float4*>(xc + (n + 1) * D);
+    const float4* pc = reinterpret_cast<const float4*>(xc);
+    const float4 r0 = pr[0], r1 = pr[1], c0 = __ldg(pc), c1 = __ldg(pc + 1);
+    uint4 v = make_uint4(pack_half2(r0.x + c0.x, r0.y + c0.y), pack_half2(r0.z + c0.z, r0.w + c0.w),
+                         pack_half2(r1.x + c1.x, r1.y + c1.y), pack_half2(r1.z + c1.z, r1.w + c1.w));
+    if (!first) {
+      const uint4 d = dst[i];
+      __half2* vh = reinterpret_cast<__half2*>(&v);
+      const __half2* dh = reinterpret_cast<const __half2*>(&d);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) vh[j] = __hmax2(vh[j], dh[j]);
+    }
+    dst[i] = v;
+    if (cls && n == 0) {
+      float4* o = reinterpret_cast<float4*>(cls + b * D + c8 * 8);
+      o[0] = c0;
+      o[1] = c1;
+    }
   }
 }
 
@@ -828,8 +863,27 @@ int udb_v1_preprocess(const udb_v1_preprocess_t* p, void* stream) {
   if (p->net_h < 4 || p->net_w < 4) { set_error("udb_v1_preprocess: bad network shape"); return 1; }
   const int gh = (p->net_h - 4) / 4 + 1, gw = (p->net_w - 4) / 4 + 1;
   const float sh = (float)p->H / (float)p->rh, sw = (float)p->W / (float)p->rw;
-  v1_preprocess_kernel<<<grid_1d((long long)p->B * gh * gw * 8), 256, 0, ST(stream)>>>(*p, gh, gw, sh, sw);
+  v1_preprocess_kernel<4, 64><<<grid_1d((long long)p->B * gh * gw * 8), 256, 0, ST(stream)>>>(*p, gh, gw, sh, sw);
   return check_launch("v1_preprocess_kernel");
+}
+
+int udb_v1_preprocess_vit(const udb_v1_preprocess_t* p, void* stream) {
+  if (p->net_h < 14 || p->net_w < 14) { set_error("udb_v1_preprocess_vit: bad network shape"); return 1; }
+  const int gh = p->net_h / 14, gw = p->net_w / 14;
+  const float sh = (float)p->H / (float)p->rh, sw = (float)p->W / (float)p->rw;
+  v1_preprocess_kernel<14, 640><<<grid_1d((long long)p->B * gh * gw * 80), 256, 0, ST(stream)>>>(*p, gh, gw, sh, sw);
+  return check_launch("v1_preprocess_vit_kernel");
+}
+
+int udb_vit_tap_f16(const float* x, void* dst, float* cls, int32_t B, int32_t T, int32_t D, int32_t first, void* stream) {
+  if (B <= 0 || T < 2 || D <= 0 || D % 8) { set_error("udb_vit_tap_f16: bad shape (B %d, T %d, D %d; D must be a multiple of 8)", B, T, D); return 1; }
+  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(cls)) & 15) {
+    set_error("udb_vit_tap_f16: pointers must be 16-byte aligned");
+    return 1;
+  }
+  const long long total = (long long)B * (T - 1) * (D / 8);
+  vit_tap_kernel<<<grid_1d(total), 256, 0, ST(stream)>>>(x, reinterpret_cast<uint4*>(dst), cls, T - 1, D, total, first);
+  return check_launch("vit_tap_kernel");
 }
 
 int udb_layernorm_any(const udb_layernorm_any_t* p, void* stream) {

@@ -89,20 +89,16 @@ def pixel_bounds(shape_constraints: dict, resolution_level: Optional[int]):
     return (resolution_level * interval + lo, (resolution_level + 1) * interval + lo)
 
 
-def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
-    """key -> shape of every tensor in the reference UniDepthV2 `state_dict()` (same names, same
-    order of magnitude as SURVEY.md section 8b), so reference checkpoints load unchanged."""
-    s = ModelSpec(config)
-    d, h = s.embed_dim, s.hidden
-    out: "OrderedDict[str, tuple]" = OrderedDict()
-    pe = "pixel_encoder."
+def vit_encoder_param_shapes(out: "OrderedDict[str, tuple]", pe: str, d: int, depth: int):
+    """The DINOv2 encoder's state-dict entries (dinov2.py:186-257; one register token slot, no registers used), added to
+    `out` under the prefix `pe`; shared by UniDepthV2 and UniDepthV1 with a ViT encoder."""
     out[pe + "cls_token"] = (1, 1, d)
     out[pe + "pos_embed"] = (1, 1 + 37 * 37, d)
     out[pe + "register_tokens"] = (1, 1, d)
     out[pe + "mask_token"] = (1, d)
     out[pe + "patch_embed.proj.weight"] = (d, 3, PATCH, PATCH)
     out[pe + "patch_embed.proj.bias"] = (d,)
-    for i in range(s.depth):
+    for i in range(depth):
         b = f"{pe}blocks.{i}."
         for nm, shp in (("norm1.weight", (d,)), ("norm1.bias", (d,)), ("attn.qkv.weight", (3 * d, d)),
                         ("attn.qkv.bias", (3 * d,)), ("attn.proj.weight", (d, d)), ("attn.proj.bias", (d,)),
@@ -112,6 +108,16 @@ def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
             out[b + nm] = shp
     out[pe + "norm.weight"] = (d,)
     out[pe + "norm.bias"] = (d,)
+
+
+def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
+    """key -> shape of every tensor in the reference UniDepthV2 `state_dict()` (same names, same
+    order of magnitude as SURVEY.md section 8b), so reference checkpoints load unchanged."""
+    s = ModelSpec(config)
+    d, h = s.embed_dim, s.hidden
+    out: "OrderedDict[str, tuple]" = OrderedDict()
+    pe = "pixel_encoder."
+    vit_encoder_param_shapes(out, pe, d, s.depth)
 
     pd = "pixel_decoder."
     out[pd + "level_embeds"] = (1, 1, 4, h)

@@ -1,4 +1,4 @@
-"""Static description of UniDepthV1 (ConvNeXt encoder) for the inference path: hyper-parameters read from the
+"""Static description of UniDepthV1 (ConvNeXt or DINOv2 ViT encoder) for the inference path: hyper-parameters read from the
 reference's config format, the parameter table under the reference's state-dict names, and the fixed-shape
 arithmetic of `infer` (reference: unidepth/models/unidepthv1/unidepthv1.py:30-46 `_paddings` / `_shapes`,
 :423-447 `build`; unidepthv1/decoder.py:465-533 `Decoder.build`; backbones/convnext.py:301-448)."""
@@ -7,6 +7,8 @@ from __future__ import annotations
 import math
 from collections import OrderedDict
 from typing import Dict, Tuple
+
+from .spec import PATCH, _VIT, vit_encoder_param_shapes
 
 CONVNEXT_ARCHS = {
     # encoder.py:127-136 (`convnext_large`): depths / dims / per-stage end indices used as `output_idx`
@@ -20,24 +22,40 @@ class V1Spec:
         m = config["model"]
         enc = m["pixel_encoder"]
         name = enc["name"]
-        if name not in CONVNEXT_ARCHS and "arch" not in enc:
-            raise NotImplementedError(f"UniDepthV1 encoder '{name}': only the ConvNeXt encoders are implemented "
-                                      "(config_v1_cnvnxtl.json); the DINOv2 V1 variant is not")
-        arch = enc.get("arch", CONVNEXT_ARCHS.get(name))       # "arch": test-only override {depths, dims}
-        self.depths = tuple(arch["depths"])
-        self.dims = tuple(arch["dims"])
-        ends, acc = [], 0
-        for d in self.depths:
-            acc += d
-            ends.append(acc)
-        self.output_idx = tuple(enc.get("output_idx", ends))   # encoder.py:131 default [3, 6, 33, 36]
-        if tuple(self.output_idx) != tuple(ends):
-            raise NotImplementedError("output_idx must be the last block of each ConvNeXt stage")
+        self.vit = name in _VIT
+        if self.vit:
+            # encoder.py:139-193: every block is an output; `depths` are the lengths of the four block ranges the decoder
+            # max-stacks (decoder.py:371-374) and every range has the embedding width
+            d, depth, heads, taps = _VIT[name]
+            self.embed_dim, self.enc_depth, self.enc_heads = d, depth, heads
+            self.output_idx = tuple(enc.get("output_idx", taps))
+            idx = (0,) + self.output_idx
+            if len(self.output_idx) != 4 or any(b <= a for a, b in zip(idx, idx[1:])) or self.output_idx[-1] != depth:
+                raise NotImplementedError(f"output_idx {list(self.output_idx)}: needs 4 increasing block indices ending at "
+                                          f"the depth ({depth})")
+            self.depths = tuple(b - a for a, b in zip(idx, idx[1:]))
+            self.dims = (d,) * 4
+        else:
+            if name not in CONVNEXT_ARCHS and "arch" not in enc:
+                raise NotImplementedError(f"UniDepthV1 encoder '{name}': only the ConvNeXt and DINOv2 ViT encoders "
+                                          "are implemented")
+            arch = enc.get("arch", CONVNEXT_ARCHS.get(name))       # "arch": test-only override {depths, dims}
+            self.depths = tuple(arch["depths"])
+            self.dims = tuple(arch["dims"])
+            ends, acc = [], 0
+            for d in self.depths:
+                acc += d
+                ends.append(acc)
+            self.output_idx = tuple(enc.get("output_idx", ends))   # encoder.py:131 default [3, 6, 33, 36]
+            if tuple(self.output_idx) != tuple(ends):
+                raise NotImplementedError("output_idx must be the last block of each ConvNeXt stage")
         self.hidden = m["pixel_decoder"]["hidden_dim"]
         self.dec_depths = tuple(m["pixel_decoder"]["depths"])    # blocks at 1/16, 1/8 (Nystrom), 1/4 (Nystrom)
         self.heads = m["num_heads"]
         self.expansion = m["expansion"]
         self.image_shape = tuple(config["data"]["image_shape"])  # fixed network input (462, 616)
+        if self.vit and (self.image_shape[0] % PATCH or self.image_shape[1] % PATCH):
+            raise NotImplementedError(f"network shape {self.image_shape} is not a multiple of the patch size {PATCH}")
         # decoder.py:489-492: token adapters read the cls tokens of the last four BLOCKS, newest first
         per_block = [c for d, c in zip(self.depths, self.dims) for _ in range(d)]
         self.cls_dims = tuple(per_block[-i - 1] for i in range(4))
@@ -66,6 +84,23 @@ def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
     s = V1Spec(config)
     out: "OrderedDict[str, tuple]" = OrderedDict()
     pe = "pixel_encoder."
+    if s.vit:
+        vit_encoder_param_shapes(out, pe, s.embed_dim, s.enc_depth)
+    else:
+        _convnext_param_shapes(out, pe, s)
+    _decoder_param_shapes(out, s)
+    return out
+
+
+def level_grid(spec: V1Spec) -> Tuple[int, int]:
+    """The decoder's common grid (decoder.py:381-392): the ViT patch grid, or the ConvNeXt pyramid's 1/16 level."""
+    if spec.vit:
+        return spec.image_shape[0] // PATCH, spec.image_shape[1] // PATCH
+    sh = [(spec.image_shape[0] - 4) // 4 + 1, (spec.image_shape[1] - 4) // 4 + 1]
+    return sh[0] // 4, sh[1] // 4
+
+
+def _convnext_param_shapes(out, pe: str, s: V1Spec):
     d0 = s.dims[0]
     out[pe + "mask_token"] = (1, d0, 1, 1)
     out[pe + "stem.0.weight"], out[pe + "stem.0.bias"] = (d0, 3, 4, 4), (d0,)
@@ -85,6 +120,8 @@ def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
             out[b + "mlp.fc2.weight"], out[b + "mlp.fc2.bias"] = (c, 4 * c), (c,)
         prev = c
 
+
+def _decoder_param_shapes(out, s: V1Spec):
     pd = "pixel_decoder."
     hid, ex = s.hidden, s.expansion
 
@@ -155,4 +192,3 @@ def param_shapes(config: dict) -> "OrderedDict[str, tuple]":
     lin(pd + "level_embed_layer.0", hid, hid)
     lin(pd + "level_embed_layer.2", hid, hid)
     ln(pd + "level_embed_layer.3", hid)
-    return out

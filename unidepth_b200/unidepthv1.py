@@ -1,4 +1,4 @@
-"""UniDepthV1 (ConvNeXt encoder) -- drop-in for the reference's inference API, running on libudb.so (sm_100a).
+"""UniDepthV1 (ConvNeXt or DINOv2 ViT encoder) -- drop-in for the reference's inference API, running on libudb.so (sm_100a).
 
 Mirrors `unidepth.models.UniDepthV1` for the inference path only (reference:
 unidepth/models/unidepthv1/unidepthv1.py:96-110 constructor, :288-373 `infer`, :375-392 `load_pretrained`,
@@ -30,8 +30,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _cabi as cabi
-from .spec_v1 import V1Spec, param_shapes, v1_paddings, v1_shapes
-from .unidepthv2 import PyTorchModelHubMixin, _HAS_HF, _register
+from .spec_v1 import V1Spec, level_grid, param_shapes, v1_paddings, v1_shapes
+from .unidepthv2 import PyTorchModelHubMixin, _HAS_HF, _register, pack_vit_blocks
 
 f16, f32 = torch.float16, torch.float32
 
@@ -148,17 +148,35 @@ class UniDepthV1(nn.Module, PyTorchModelHubMixin,
             T[dst + "gamma"] = c32(sd[f"{src}gamma"])
 
         # ---- encoder
-        T["stem_w"] = h16(zpad(sd[pe + "stem.0.weight"].reshape(s.dims[0], 48), s.dims[0], 64))
-        T["stem_b"] = c32(sd[pe + "stem.0.bias"])
-        T["stem_ln_w"], T["stem_ln_b"] = c32(sd[pe + "stem.1.weight"]), c32(sd[pe + "stem.1.bias"])
-        for i, depth in enumerate(s.depths):
-            st = f"{pe}stages.{i}."
-            if i > 0:
-                w = sd[st + "downsample.1.weight"]                               # [C, Cp, 2, 2] -> [C, (dy,dx,ci)]
-                T[f"ds{i}.ln_w"], T[f"ds{i}.ln_b"] = c32(sd[st + "downsample.0.weight"]), c32(sd[st + "downsample.0.bias"])
-                T[f"ds{i}.w"], T[f"ds{i}.b"] = h16(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1)), c32(sd[st + "downsample.1.bias"])
-            for j in range(depth):
-                block(f"s{i}.b{j}.", f"{st}blocks.{j}.", ("conv_dw", "norm", "mlp.fc1", "mlp.fc2"))
+        hc, wc = level_grid(s)
+        if s.vit:
+            d = s.embed_dim
+            T["patch_w"] = h16(zpad(sd[pe + "patch_embed.proj.weight"].reshape(d, 588).float(), d, 640))
+            T["patch_b"], T["cls"] = c32(sd[pe + "patch_embed.proj.bias"]), c32(sd[pe + "cls_token"].reshape(d))
+            # dinov2.py:267-304 with interpolate_offset 0.1 (unidepthv1.py:418-424): the bicubic resampling of the 37x37
+            # table takes its sample positions from the scale factor; the network shape is fixed, so the resampled table
+            # is a constant of the weights, folded here with the reference's own call
+            pos = sd[pe + "pos_embed"].float()
+            m = math.isqrt(pos.shape[1] - 1)
+            grid = F.interpolate(pos[:, 1:].reshape(1, m, m, d).permute(0, 3, 1, 2), mode="bicubic", antialias=False,
+                                 scale_factor=((hc + 0.1) / m, (wc + 0.1) / m))
+            assert tuple(grid.shape[-2:]) == (hc, wc), grid.shape
+            T["pos"] = c32(torch.cat([pos[0, :1], grid.permute(0, 2, 3, 1).reshape(hc * wc, d)], 0))
+            for i, blk in enumerate(pack_vit_blocks(sd, pe, s.enc_depth)):
+                for k, v in blk.items():
+                    T[f"blocks.{i}.{k}"] = v
+        else:
+            T["stem_w"] = h16(zpad(sd[pe + "stem.0.weight"].reshape(s.dims[0], 48), s.dims[0], 64))
+            T["stem_b"] = c32(sd[pe + "stem.0.bias"])
+            T["stem_ln_w"], T["stem_ln_b"] = c32(sd[pe + "stem.1.weight"]), c32(sd[pe + "stem.1.bias"])
+            for i, depth in enumerate(s.depths):
+                st = f"{pe}stages.{i}."
+                if i > 0:
+                    w = sd[st + "downsample.1.weight"]                               # [C, Cp, 2, 2] -> [C, (dy,dx,ci)]
+                    T[f"ds{i}.ln_w"], T[f"ds{i}.ln_b"] = c32(sd[st + "downsample.0.weight"]), c32(sd[st + "downsample.0.bias"])
+                    T[f"ds{i}.w"], T[f"ds{i}.b"] = h16(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1)), c32(sd[st + "downsample.1.bias"])
+                for j in range(depth):
+                    block(f"s{i}.b{j}.", f"{st}blocks.{j}.", ("conv_dw", "norm", "mlp.fc1", "mlp.fc2"))
 
         # ---- decoder: adapters, embeddings
         for l in range(4):
@@ -170,10 +188,6 @@ class UniDepthV1(nn.Module, PyTorchModelHubMixin,
             T[f"tok.{l}.w"], T[f"tok.{l}.b"] = c32(sd[t + ".1.weight"]), c32(sd[t + ".1.bias"])
         # level embedding MLP of the four learned level vectors + sine position embedding of the common grid
         # (decoder.py:410-433): constants of (weights, network shape), folded once here
-        sh = [(s.image_shape[0] - 4) // 4 + 1, (s.image_shape[1] - 4) // 4 + 1]
-        for _ in range(2):
-            sh = [sh[0] // 2, sh[1] // 2]
-        hc, wc = sh
         le = F.linear(F.gelu(F.linear(sd[pd + "level_embeds"].float(), sd[pd + "level_embed_layer.0.weight"].float(),
                                       sd[pd + "level_embed_layer.0.bias"].float())),
                       sd[pd + "level_embed_layer.2.weight"].float(), sd[pd + "level_embed_layer.2.bias"].float())
@@ -305,7 +319,11 @@ class UniDepthV1(nn.Module, PyTorchModelHubMixin,
         if self._engine is not None:
             return self._engine
         handle = C.c_void_p()
-        cabi.check(cabi.lib().udb_v1_create(C.byref(self._engine_config()), C.byref(handle)), "udb_v1_create")
+        if self.spec.vit:
+            cabi.check(cabi.lib().udb_v1_create_vit(C.byref(self._engine_config()), self.spec.enc_heads, C.byref(handle)),
+                       "udb_v1_create_vit")
+        else:
+            cabi.check(cabi.lib().udb_v1_create(C.byref(self._engine_config()), C.byref(handle)), "udb_v1_create")
         for name, t in P["T"].items():
             assert t.is_cuda, name
         self._register(handle, P["T"], P["S"])

@@ -49,6 +49,53 @@ class _Node(nn.Module):
     """Anonymous container used to reproduce the reference's dotted parameter names."""
 
 
+def _enc16(w: torch.Tensor, split: bool) -> torch.Tensor:
+    """Encoder GEMM weight [N, K]: f16, or in split mode [N, 3K] = [hi | hi | lo] with w ~= hi + lo."""
+    w = w.to(f32)
+    hi = w.to(f16)
+    if not split:
+        return hi.contiguous()
+    lo = (w - hi.to(f32)).to(f16)
+    return torch.cat([hi, hi, lo], dim=1).contiguous()
+
+
+def _ln_fold(w, b, lnw, lnb):
+    """LayerNorm folded into the Linear that follows it:  LN(x) W^T + b = rstd (x W'^T - mean c1) + c2  with
+    W' = W diag(ln_w) (f16, what the MMA multiplies), c1 = row sums of the ROUNDED W', c2 = W ln_b + b."""
+    w, b, lnw, lnb = w.float(), b.float(), lnw.float(), lnb.float()
+    wf = (w * lnw.unsqueeze(0)).to(f16)
+    return wf.contiguous(), wf.float().sum(dim=1).contiguous(), (w @ lnb + b).contiguous()
+
+
+def pack_vit_blocks(sd: dict, pe: str, depth: int, split: bool = False, fuse: bool = False) -> list:
+    """Per-block operand dicts of a DINOv2 encoder (state dict `sd`, prefix `pe`), the names the engines' shared block
+    (engine_common.h `vit_block`) reads as blocks.<i>.<name>: default f16, split precision or fused LayerNorm."""
+    h16 = lambda t: t.to(f16).contiguous()
+    c32 = lambda t: t.to(f32).contiguous()
+    enc16 = lambda w: _enc16(w, split)
+    blocks = []
+    for i in range(depth):
+        b = f"{pe}blocks.{i}."
+        if fuse:
+            qw, qc1, qc2 = _ln_fold(sd[b + "attn.qkv.weight"], sd[b + "attn.qkv.bias"], sd[b + "norm1.weight"], sd[b + "norm1.bias"])
+            fw, fc1, fc2 = _ln_fold(sd[b + "mlp.fc1.weight"], sd[b + "mlp.fc1.bias"], sd[b + "norm2.weight"], sd[b + "norm2.bias"])
+            blocks.append(dict(
+                qkv_wf=qw, qkv_c1=qc1, qkv_c2=qc2, fc1_wf=fw, fc1_c1=fc1, fc1_c2=fc2,
+                proj_w=h16(sd[b + "attn.proj.weight"]), proj_b=c32(sd[b + "attn.proj.bias"]), ls1=c32(sd[b + "ls1.gamma"]),
+                fc2_w=h16(sd[b + "mlp.fc2.weight"]), fc2_b=c32(sd[b + "mlp.fc2.bias"]), ls2=c32(sd[b + "ls2.gamma"])))
+            continue
+        blocks.append(dict(
+            n1w=c32(sd[b + "norm1.weight"]), n1b=c32(sd[b + "norm1.bias"]),
+            qkv_w=enc16(sd[b + "attn.qkv.weight"]), qkv_b=c32(sd[b + "attn.qkv.bias"]),
+            proj_w=enc16(sd[b + "attn.proj.weight"]), proj_b=c32(sd[b + "attn.proj.bias"]),
+            ls1=c32(sd[b + "ls1.gamma"]),
+            n2w=c32(sd[b + "norm2.weight"]), n2b=c32(sd[b + "norm2.bias"]),
+            fc1_w=enc16(sd[b + "mlp.fc1.weight"]), fc1_b=c32(sd[b + "mlp.fc1.bias"]),
+            fc2_w=enc16(sd[b + "mlp.fc2.weight"]), fc2_b=c32(sd[b + "mlp.fc2.bias"]),
+            ls2=c32(sd[b + "ls2.gamma"])))
+    return blocks
+
+
 def _register(root: nn.Module, dotted: str, tensor: torch.Tensor):
     parts = dotted.split(".")
     mod = root
@@ -169,24 +216,7 @@ class UniDepthV2(nn.Module, PyTorchModelHubMixin,
             raise ValueError(f"precision must be 'f16' or 'split', not {self.precision!r}")
         split = self.precision == "split"
 
-        def enc16(w):
-            """Encoder GEMM weight [N, K]: f16, or in split mode [N, 3K] = [hi | hi | lo] with w ~= hi + lo."""
-            w = w.to(f32)
-            hi = w.to(f16)
-            if not split:
-                return hi.contiguous()
-            lo = (w - hi.to(f32)).to(f16)
-            return torch.cat([hi, hi, lo], dim=1).contiguous()
-
         fuse = self._fuse()
-
-        def ln_fold(w, b, lnw, lnb):
-            """LayerNorm folded into the Linear that follows it:  LN(x) W^T + b = rstd (x W'^T - mean c1) + c2  with
-            W' = W diag(ln_w) (f16, what the MMA multiplies), c1 = row sums of the ROUNDED W', c2 = W ln_b + b."""
-            w, b, lnw, lnb = w.float(), b.float(), lnw.float(), lnb.float()
-            wf = (w * lnw.unsqueeze(0)).to(f16)
-            return wf.contiguous(), wf.float().sum(dim=1).contiguous(), (w @ lnb + b).contiguous()
-
         P: dict = {"split": split, "fuse_ln": fuse}
         d, hid = s.embed_dim, s.hidden
         # The attention kernel works on 64-wide heads.  Narrower decoder heads (ViT-S: 256/8 = 32) are
@@ -210,29 +240,10 @@ class UniDepthV2(nn.Module, PyTorchModelHubMixin,
         pe = "pixel_encoder."
         wpe = torch.zeros((d, 640), device=dev, dtype=f32)
         wpe[:, :588] = sd[pe + "patch_embed.proj.weight"].reshape(d, 588).to(f32)
-        P["patch_w"], P["patch_b"] = enc16(wpe), c32(sd[pe + "patch_embed.proj.bias"])
+        P["patch_w"], P["patch_b"] = _enc16(wpe, split), c32(sd[pe + "patch_embed.proj.bias"])
         P["cls"] = c32(sd[pe + "cls_token"].reshape(d))
         P["pos"] = c32(sd[pe + "pos_embed"].reshape(-1, d))
-        P["blocks"] = []
-        for i in range(s.depth):
-            b = f"{pe}blocks.{i}."
-            if fuse:
-                qw, qc1, qc2 = ln_fold(sd[b + "attn.qkv.weight"], sd[b + "attn.qkv.bias"], sd[b + "norm1.weight"], sd[b + "norm1.bias"])
-                fw, fc1, fc2 = ln_fold(sd[b + "mlp.fc1.weight"], sd[b + "mlp.fc1.bias"], sd[b + "norm2.weight"], sd[b + "norm2.bias"])
-                P["blocks"].append(dict(
-                    qkv_wf=qw, qkv_c1=qc1, qkv_c2=qc2, fc1_wf=fw, fc1_c1=fc1, fc1_c2=fc2,
-                    proj_w=h16(sd[b + "attn.proj.weight"]), proj_b=c32(sd[b + "attn.proj.bias"]), ls1=c32(sd[b + "ls1.gamma"]),
-                    fc2_w=h16(sd[b + "mlp.fc2.weight"]), fc2_b=c32(sd[b + "mlp.fc2.bias"]), ls2=c32(sd[b + "ls2.gamma"])))
-                continue
-            P["blocks"].append(dict(
-                n1w=c32(sd[b + "norm1.weight"]), n1b=c32(sd[b + "norm1.bias"]),
-                qkv_w=enc16(sd[b + "attn.qkv.weight"]), qkv_b=c32(sd[b + "attn.qkv.bias"]),
-                proj_w=enc16(sd[b + "attn.proj.weight"]), proj_b=c32(sd[b + "attn.proj.bias"]),
-                ls1=c32(sd[b + "ls1.gamma"]),
-                n2w=c32(sd[b + "norm2.weight"]), n2b=c32(sd[b + "norm2.bias"]),
-                fc1_w=enc16(sd[b + "mlp.fc1.weight"]), fc1_b=c32(sd[b + "mlp.fc1.bias"]),
-                fc2_w=enc16(sd[b + "mlp.fc2.weight"]), fc2_b=c32(sd[b + "mlp.fc2.bias"]),
-                ls2=c32(sd[b + "ls2.gamma"])))
+        P["blocks"] = pack_vit_blocks(sd, pe, s.depth, split, fuse)
         P["norm_w"], P["norm_b"] = c32(sd[pe + "norm.weight"]), c32(sd[pe + "norm.bias"])
 
         pd = "pixel_decoder."
